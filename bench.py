@@ -5,7 +5,8 @@ other configs of the metric (MViTv2-S, X3D-M, MaskFeat-S, MaskFeat on MViTv2-B 3
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
-    python bench.py --impl reference ...     # the UNMODIFIED reference (baseline/_ref) on the box's host cores
+    python bench.py --impl reference ...     # the UNMODIFIED reference (oracle/_ref) on the box's host cores
+    python bench.py ... --dump-outputs DIR   # also write the headline leg's last timed step's outputs as DIR/*.npy
 
 A step = zero_grad -> forward (engine kernels) -> loss -> backward (engine kernels) -> [one NCCL all-reduce of the flat
 gradient bucket when N > 1] -> optimizer step, on the recipe's per-GPU batch of synthetic Kinetics-shaped input, random
@@ -130,11 +131,11 @@ REF_YAML = {"SLOWFAST_8x8_R50": "Kinetics/SLOWFAST_8x8_R50.yaml", "MVITv2_S_16x4
 
 
 def reference_model(preset: str, overrides=()):
-    """The UNMODIFIED reference module (slowfast.models.build_model on the reference's own yaml) from baseline/_ref (or the
-    build container's checkout) through oracle/refshim.py.  Returns (cfg, model) or raises if no reference tree exists."""
+    """The UNMODIFIED reference module (slowfast.models.build_model on the reference's own yaml) from oracle/_ref (copied
+    there by build()) through oracle/refshim.py.  Returns (cfg, model) or raises if no reference tree exists."""
     from oracle import refshim
     if not refshim.reference_available():
-        raise RuntimeError("no reference tree (run baseline/install_ref.sh in the build container)")
+        raise RuntimeError("no reference tree (build() copies it into oracle/_ref when a checkout is readable)")
     cfg = refshim.load_cfg(REF_YAML[preset], list(overrides))
     return cfg, refshim.build_reference_model(cfg)
 
@@ -178,7 +179,7 @@ def time_reference_cpu(preset: str, batch: int, steps: int, warm: int, budget_s:
 
 def reference_arm(args):
     """``--impl reference``: the reference's OWN CPU implementation of the path (its nn.Conv3d / BatchNorm3d / ... modules,
-    unmodified, from baseline/_ref) on this box's host cores, all the threads the process may use, on the same workload
+    unmodified, from oracle/_ref) on this box's host cores, all the threads the process may use, on the same workload
     (SlowFast-8x8-R50 train step, the same per-step batch); steps are bounded so that the run ends within minutes."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -197,7 +198,7 @@ def reference_arm(args):
                 dtype="f32", data="synthetic", impl="reference",
                 config=dict(workload=leg["what"], per_gpu_batch=args.batch, global_batch=args.batch,
                             parallelism="host CPU", threads=r["threads"],
-                            note="unmodified reference modules (baseline/_ref) on the host cores; fwd + CE + bwd, no "
+                            note="unmodified reference modules (oracle/_ref) on the host cores; fwd + CE + bwd, no "
                                  "optimizer step"),
                 cpu_baseline=dict(value=v, unit="clips/s", cores=r["threads"], kind=kind,
                                   sample=f"{r['steps']} x fwd+bwd of {args.batch} clips through slowfast.models.build_model "
@@ -297,26 +298,59 @@ def build_leg(name: str, nsplit: int, dev, rank: int, batch=None):
     labels = labels.pin_memory()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     meta = torch.Tensor()
+    last = {}   # the model output of the latest step (--dump-outputs)
 
     def step(x, y):
         opt.zero_grad(set_to_none=True)
         if mname == "MaskMViT":
             preds, labs = model([x[0], meta, x[1]])
+            last["logits"] = preds[0]
             loss = sum(F.mse_loss(p, l[0]) * l[1] for p, l in zip(preds, labs))   # losses.py:38-62 MultipleMSELoss
         else:
-            loss = F.cross_entropy(model(x), y)
+            last["logits"] = model(x)
+            loss = F.cross_entropy(last["logits"], y)
         loss.backward()
         if world > 1:
             model.allreduce_gradients()
         opt.step()
         return loss
 
-    return dict(name=name, cfg=cfg, model=model, step=step, host=host, labels=labels, B=B, leg=leg)
+    return dict(name=name, cfg=cfg, model=model, step=step, host=host, labels=labels, B=B, leg=leg, last=last)
 
 
-def measure_leg(L, args, dev, world, barrier, max_over_ranks, clock_index=None):
+DUMP_SAMPLE = 1 << 21   # parameter / gradient elements written by --dump-outputs (8 MiB each in float32)
+
+
+def dump_outputs(out_dir: str, model, loss, logits) -> None:
+    """What the caller of a training step receives, as float32 .npy files: the loss, the logits, and the same seeded
+    sample of DUMP_SAMPLE elements of the updated parameters and of their gradients (all parameters flattened in
+    model.parameters() order; all of them when there are fewer).  The kernels accumulate some sums with atomics, so two
+    runs agree to rounding, not bit for bit: compare with a tolerance (two runs of the 10 + 3 step headline on a B200 at
+    1000 W: loss 8e-7, logits 1e-5, parameters 2e-6, gradients 4e-3 relative L2)."""
+    import numpy as np
+    params = list(model.parameters())
+    if getattr(model, "flat_grad_only", False):   # no param.grad: read the bucket where FlatOptimizer reads it
+        from slowfast_b200.engine import flat_offsets
+        offsets, _ = flat_offsets(params)
+        grads = [model.ctx.flat_grad[o:o + p.numel()] for p, o in zip(params, offsets)]
+    else:
+        grads = [p.grad for p in params]
+    flat_p = torch.cat([p.detach().flatten() for p in params])
+    flat_g = torch.cat([g.detach().flatten() for g in grads])
+    n = flat_p.numel()
+    idx = torch.arange(n) if n <= DUMP_SAMPLE else \
+        torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+    idx = idx.to(flat_p.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("loss", loss.detach().reshape(1)), ("logits", logits.detach()),
+                    ("params_sample", flat_p[idx]), ("grads_sample", flat_g[idx])):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
+def measure_leg(L, args, dev, world, barrier, max_over_ranks, clock_index=None, dump_dir=None):
     """(1) device-resident clips/s, (2) end-to-end clips/s with pinned H2D + loss read-back inside the timed region,
-    (3) per-class roofline of the implicit-GEMM kernels.  Returns a dict."""
+    (3) per-class roofline of the implicit-GEMM kernels.  With ``dump_dir``, the outputs of the last step of (1) are
+    written there before anything else runs.  Returns a dict."""
     from slowfast_b200 import ops
     step, host, labels_h, B = L["step"], L["host"], L["labels"], L["B"]
     resident = [t.to(dev) for t in host]
@@ -339,6 +373,8 @@ def measure_leg(L, args, dev, world, barrier, max_over_ranks, clock_index=None):
     launches = ops.launches() - l0
     clocks = sampler.stop() if sampler else None
     value = B * world * args.steps / (ms_total * 1e-3)
+    if dump_dir:
+        dump_outputs(dump_dir, L["model"], loss, L["last"]["logits"])
 
     # end to end through the public call with HOST buffers: pinned H2D every step (prefetched on a copy stream, as a
     # loader with non_blocking copies does) + D2H read of the loss every step
@@ -518,7 +554,7 @@ def profile_conv_kernels(model, step, resident, labels, peaks, leg_name):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--nsplit", type=int, default=3, choices=[1, 3])
@@ -530,7 +566,12 @@ def main():
                     help="skip timing the reference's own modules (ATen / cuDNN) on this GPU (N=1 only)")
     ap.add_argument("--torch-optim", action="store_true",
                     help="step torch.optim.SGD / AdamW on param.grad instead of the fused flat-bucket optimizer")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, logits and a seeded sample of the updated parameters and their gradients "
+                         "after the headline leg's last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global TORCH_OPTIM
     TORCH_OPTIM = args.torch_optim
     if args.impl == "reference":
@@ -567,7 +608,8 @@ def main():
     peaks = load_peaks()
     # ---- headline: SlowFast-8x8-R50 ------------------------------------------------------------------------------
     L = build_leg("slowfast", args.nsplit, dev, rank, batch=args.batch)
-    head = measure_leg(L, args, dev, world, barrier, max_over_ranks, clock_index=local if rank == 0 else None)
+    head = measure_leg(L, args, dev, world, barrier, max_over_ranks, clock_index=local if rank == 0 else None,
+                       dump_dir=args.dump_outputs if rank == 0 else None)
     cfg = L["cfg"]
     del L
     torch.cuda.empty_cache()
@@ -579,7 +621,7 @@ def main():
             r = time_reference_cpu("SLOWFAST_8x8_R50", 4, steps=3, warm=1, budget_s=25.0)
             cpu_baseline = dict(value=r["clips_per_s"], unit="clips/s", cores=r["threads"], kind="reference",
                                 sample=f"{r['steps']} x fwd+CE+bwd of {r['batch']} clips through the unmodified reference "
-                                       f"modules (baseline/_ref, fp32 ATen CPU kernels), {r['ms_per_step']:.0f} ms/step")
+                                       f"modules (oracle/_ref, fp32 ATen CPU kernels), {r['ms_per_step']:.0f} ms/step")
         except Exception as e:  # noqa: BLE001
             cpu_baseline = dict(error=repr(e)[:300])
 

@@ -82,6 +82,23 @@ def digest(t: torch.Tensor):
     return dict(norm=f.norm().item(), sum=f.sum().item(), head=f[:4].tolist(), numel=f.numel())
 
 
+LABELS_WHOLE = 100000   # HOG targets up to this many values are stored whole; larger ones as a seeded sample of rows
+LABELS_SAMPLED = 50000  # (so that a golden file stays under 1 MB)
+
+
+def store_labels(gold, labels: torch.Tensor) -> None:
+    """``labels``, or for large targets a fixed seeded sample of its rows (``label_rows``), plus the digest of all."""
+    labels = labels.detach()
+    gold["labels_digest"] = digest(labels)
+    if labels.numel() <= LABELS_WHOLE:
+        gold["labels"] = labels.clone()
+        return
+    k = max(1, LABELS_SAMPLED // labels[0].numel())
+    rows = torch.randperm(labels.shape[0], generator=torch.Generator().manual_seed(0))[:k].sort().values
+    gold["label_rows"] = rows
+    gold["labels"] = labels[rows].clone()
+
+
 def run_case(name, yaml, overrides, batch, in_seed, st_seed):
     if isinstance(overrides, str):
         overrides = NAMED_OVERRIDES[overrides]
@@ -155,8 +172,7 @@ def run_case(name, yaml, overrides, batch, in_seed, st_seed):
         print(f"[{name}] reference fp32 vs fp64: logits {gold['logits_env']:.2e}; sampled-gradient rel-L2 median "
               f"{e[len(e) // 2]:.2e} max {e[-1]:.2e}")
     if ref_labels is not None:
-        gold["labels"] = ref_labels.detach().clone() if ref_labels.numel() < 200000 else None
-        gold["labels_digest"] = digest(ref_labels)
+        store_labels(gold, ref_labels)
     out = os.path.join(ROOT, "tests", "golden", name + ".pt")
     torch.save(gold, out)
     print(f"[{name}] wrote {out} ({os.path.getsize(out) / 1024:.1f} KiB)")

@@ -1,12 +1,12 @@
 """TEST INFRASTRUCTURE — never imported by the product path.
 
-Makes the UNMODIFIED reference (facebookresearch/SlowFast, mounted read-only at /root/reference in the build
-container) importable offline by providing tiny stand-ins for its un-vendored Python dependencies (fvcore, iopath,
+Makes the UNMODIFIED reference (facebookresearch/SlowFast, copied into oracle/_ref by build() through
+oracle/install_ref.py) importable offline by providing tiny stand-ins for its un-vendored Python dependencies (fvcore, iopath,
 pytorchvideo, detectron2, simplejson, matplotlib, av) and the ``vision.fair.slowfast`` namespace its tools import
 (SURVEY.md §8b/§8c).  Used only to (a) pin ``oracle/torch_oracle.py`` against the reference's own modules and
 (b) generate the golden fixtures under ``tests/golden``, (c) run the reference itself as the CPU / ATen-GPU baseline of
-``bench.py`` and in the driver tests (tools/train_net.py, test_net.py).  /root/reference does not exist on the GPU box;
-``baseline/_ref`` (installed by ``baseline/install_ref.sh``, byte-identical python files) does.
+``bench.py`` and in the driver tests (tools/train_net.py, test_net.py).  oracle/_ref is git-ignored and travels with the
+built tree; ``baseline/_ref`` (installed by ``baseline/install_ref.sh``, byte-identical python files) is also searched.
 
 The stand-ins restate published behaviour of those packages:
   fvcore.nn.weight_init.c2_msra_fill  = kaiming_normal_(mode="fan_out", nonlinearity="relu"), bias 0
@@ -28,9 +28,10 @@ _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _find_reference_root() -> str:
-    """The unmodified reference: $SLOWFAST_REFERENCE_ROOT, else the read-only checkout of the build container, else the
-    offline install made by baseline/install_ref.sh (git-ignored; it travels to the GPU box with the snapshot)."""
-    cands = [os.environ.get("SLOWFAST_REFERENCE_ROOT"), "/root/reference", os.path.join(_REPO, "baseline", "_ref")]
+    """The unmodified reference: $SLOWFAST_REFERENCE_ROOT, else the copy build() makes in oracle/_ref
+    (oracle/install_ref.py), else the offline install made by baseline/install_ref.sh (both git-ignored)."""
+    cands = [os.environ.get("SLOWFAST_REFERENCE_ROOT"), os.path.join(_REPO, "oracle", "_ref"),
+             os.path.join(_REPO, "baseline", "_ref")]
     for c in cands:
         if c and os.path.isdir(os.path.join(c, "slowfast")) and os.path.isdir(os.path.join(c, "configs")):
             return c
@@ -361,7 +362,7 @@ def install() -> None:
     if _installed:
         return
     if not reference_available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT} (it only exists in the build container)")
+        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT} (build() installs it when a checkout is readable)")
     _install_fvcore()
     _install_misc()
     for name in ("vision", "vision.fair", "vision.fair.slowfast"):

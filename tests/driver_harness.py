@@ -2,8 +2,8 @@
 ``test(cfg)``) on a synthetic dataset, with either the stock models or the engine's drop-ins behind
 ``slowfast.models.build_model``.
 
-The reference tree comes from ``oracle/refshim.py`` (the build container's read-only checkout, or the byte-identical
-offline install under baseline/_ref on the GPU box).  Nothing in the reference is edited; the harness only
+The reference tree comes from ``oracle/refshim.py`` (the byte-identical copy build() makes in oracle/_ref, or the
+offline install under baseline/_ref).  Nothing in the reference is edited; the harness only
   * registers a ``Synthetic`` dataset class in the reference's DATASET_REGISTRY (its designated extension point,
     slowfast/datasets/build.py:8-13) and selects it with TRAIN.DATASET / TEST.DATASET,
   * calls ``slowfast_b200.integration.register(replace=True)`` (INTEGRATION.md section 2),

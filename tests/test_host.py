@@ -52,28 +52,45 @@ def test_slowfast_state_dict_matches_reference_keys():
     assert n_bn == 110
 
 
-def test_slowfast_init_is_bit_identical_to_reference_when_available():
+def _reference_init(yaml, overrides=()):
+    """The reference's resolved config and the digests of its freshly initialised state (oracle/make_golden_reference.py)."""
+    from oracle.make_golden_reference import init_key
+    return torch.load(os.path.join(GOLDEN, "reference_init.pt"))[init_key(yaml, list(overrides))]
+
+
+def _reference_cfg(yaml, ref, overrides=()):
+    """The reference's own CfgNode when the reference is installed (oracle/_ref), else its stored resolved values."""
     from oracle import refshim
-    if not refshim.reference_available():
-        pytest.skip("/root/reference is not present on this box")
+    from slowfast_b200.config import Cfg
+    if refshim.reference_available():
+        return refshim.load_cfg(yaml, list(overrides))
+    return Cfg(ref["cfg"])
+
+
+def _assert_same_init(state, ref):
+    from oracle.make_golden_reference import layout_digest, tensor_digest
+    assert layout_digest(state) == ref["layout"], "state_dict names / shapes / order differ from the reference's"
+    bad = [k for i, (k, v) in enumerate(state.items()) if tensor_digest(v) != ref["values"][8 * i:8 * i + 8]]
+    assert not bad, bad[:5]
+
+
+def test_slowfast_init_is_bit_identical_to_reference_when_available():
+    """Same seed, same initial weights as the reference's build_model, compared through the digests of its state."""
     from slowfast_b200.config import get_cfg
     from slowfast_b200.nets.resnet import B200SlowFast
-    rcfg = refshim.load_cfg("Kinetics/SLOWFAST_8x8_R50.yaml")
-    ref = refshim.build_reference_model(rcfg).state_dict()
-    torch.manual_seed(rcfg.RNG_SEED)
-    mine = B200SlowFast(get_cfg("SLOWFAST_8x8_R50")).state_dict()
-    assert all(torch.equal(mine[k], ref[k]) for k in ref)
-    # and the engine classes accept the reference's own CfgNode
-    torch.manual_seed(rcfg.RNG_SEED)
-    mine2 = B200SlowFast(rcfg).state_dict()
-    assert all(torch.equal(mine2[k], ref[k]) for k in ref)
+    ref = _reference_init("Kinetics/SLOWFAST_8x8_R50.yaml")
+    torch.manual_seed(ref["cfg"]["RNG_SEED"])
+    _assert_same_init(B200SlowFast(get_cfg("SLOWFAST_8x8_R50")).state_dict(), ref)
+    # and the engine classes accept the reference's own resolved config
+    torch.manual_seed(ref["cfg"]["RNG_SEED"])
+    _assert_same_init(B200SlowFast(_reference_cfg("Kinetics/SLOWFAST_8x8_R50.yaml", ref)).state_dict(), ref)
 
 
 def test_integration_registers_into_reference_registry():
     """slowfast.models.build_model (the unmodified reference) hands out the engine class after register()."""
     from oracle import refshim
     if not refshim.reference_available():
-        pytest.skip("/root/reference is not present on this box")
+        pytest.skip("no reference tree (build() copies it into oracle/_ref when a checkout is readable)")
     refshim.install()
     import slowfast_b200.integration as integ
     from slowfast.models import build_model
@@ -139,25 +156,18 @@ def test_state_dict_matches_reference_keys(gold_name):
 
 @pytest.mark.parametrize("gold_name", sorted(MODELS))
 def test_init_is_bit_identical_to_reference_when_available(gold_name):
-    from oracle import refshim
-    if not refshim.reference_available():
-        pytest.skip("/root/reference is not present on this box")
     from slowfast_b200.config import get_cfg
     preset, yaml, spec = MODELS[gold_name]
     ov = EXTRA_OVERRIDES.get(gold_name, [])
-    rcfg = refshim.load_cfg(yaml, ov)
-    ref = refshim.build_reference_model(rcfg).state_dict()
-    torch.manual_seed(rcfg.RNG_SEED)
+    ref = _reference_init(yaml, ov)
+    torch.manual_seed(ref["cfg"]["RNG_SEED"])
     cfg = get_cfg(preset)
     for k, v in zip(ov[0::2], ov[1::2]):
         sec, key = k.split(".")
         cfg[sec][key] = v
-    mine = _engine_class(spec)(cfg).state_dict()
-    bad = [k for k in ref if not torch.equal(mine[k], ref[k])]
-    assert not bad, bad[:5]
-    torch.manual_seed(rcfg.RNG_SEED)
-    mine2 = _engine_class(spec)(rcfg).state_dict()  # the reference's own CfgNode is accepted as-is
-    assert all(torch.equal(mine2[k], ref[k]) for k in ref)
+    _assert_same_init(_engine_class(spec)(cfg).state_dict(), ref)
+    torch.manual_seed(ref["cfg"]["RNG_SEED"])
+    _assert_same_init(_engine_class(spec)(_reference_cfg(yaml, ref, ov)).state_dict(), ref)  # the reference's config as-is
 
 
 def test_x3d_widths_and_parameter_count():
@@ -178,21 +188,15 @@ MORE_YAMLS = ["Kinetics/SLOW_8x8_R50.yaml", "Kinetics/SLOW_4x16_R50.yaml", "Kine
 
 @pytest.mark.parametrize("yaml", MORE_YAMLS)
 def test_engine_accepts_other_reference_yamls(yaml):
-    """The engine classes are built straight from the reference's own CfgNode for the other shipped recipes of the
+    """The engine classes are built straight from the reference's resolved config for the other shipped recipes of the
     same model families (Slow / I3D / R101, SlowFast 4x16, X3D-XS/S/L, MViTv2-B, MaskFeat MViTv2-L): identical
     state_dict (names, order, shapes) and bit-identical initialisation under the same seed."""
-    from oracle import refshim
-    if not refshim.reference_available():
-        pytest.skip("/root/reference is not present on this box")
     from slowfast_b200.integration import ENGINE_CLASSES, _resolve
-    rcfg = refshim.load_cfg(yaml)
-    ref = refshim.build_reference_model(rcfg).state_dict()
+    ref = _reference_init(yaml)
+    rcfg = _reference_cfg(yaml, ref)
     cls = _resolve(ENGINE_CLASSES[rcfg.MODEL.MODEL_NAME])
     torch.manual_seed(rcfg.RNG_SEED)
-    mine = cls(rcfg).state_dict()
-    assert [(k, tuple(v.shape)) for k, v in mine.items()] == [(k, tuple(v.shape)) for k, v in ref.items()]
-    bad = [k for k in ref if not torch.equal(mine[k], ref[k])]
-    assert not bad, bad[:5]
+    _assert_same_init(cls(rcfg).state_dict(), ref)
 
 
 def test_kernel_selection_predicates_without_a_gpu():
